@@ -3,6 +3,7 @@
 
   python bench.py --gpus 1 --steps K --warmup W            (N>1: launched by torch.distributed.run)
   python bench.py --impl reference ...                      (the reference algorithm on the host cores)
+  python bench.py ... --dump-outputs DIR                    (also writes the last timed step's corrected reads: dump_outputs)
 
 Workload (BASELINE.json configs[2], "cfg3", the one the metric is quoted on; it fits one GPU): ONE synthetic
 read set of 50k reads x 20 kb, R10 error profile, ~40x, `-b 128`, W = 4096.  The job is that set: its target
@@ -29,6 +30,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -62,6 +64,8 @@ def parse():
                     "256-target launches 800-868 Mbases/s, 500: 785-796, 1000: 709, 2000: 584 - smaller launches overlap better across the lanes)")
     ap.add_argument("--host-windowing", action="store_true", help="e2e region submits host-computed OverlapWindows (hb_submit_target) instead of raw alignments")
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU legs (cpu_baseline / --impl reference); 0 = all host threads")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the corrected reads of the last timed step (rank 0's share) as .npy "
+                    "files under DIR (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -221,11 +225,40 @@ def workload_name(args):
             f"-b {args.batch_size}")
 
 
-def ensure_model():
-    from herro_b200 import weights as hbw
-    d = os.path.join(ROOT, "tests", "_tmp")
+DUMP_SAMPLE_BASES = 8 << 20  # corrected bases written by dump_outputs: 32 MB as float32
+
+
+def dump_outputs(d, segments):
+    """What a caller of the timed path received for the last timed step, as float .npy files under `d`:
+      target_ids           [T] f64  targets that produced a record, ascending
+      segments_per_target  [T] f64  0 = the read is omitted from the output
+      segment_lengths      [S] f64  every segment of those targets, in target order
+      sample_target_ids    [k] f64  a fixed, seeded sample of target_ids whose bases fit DUMP_SAMPLE_BASES
+      sample_bases         [B] f32  ASCII codes of the sampled targets' segments back to back, in sample order
+    `segments`: {target id: list of bytes (empty or None = omitted)}."""
     os.makedirs(d, exist_ok=True)
-    p = os.path.join(d, f"bench_model_{os.getpid()}.hbw")
+    rids = sorted(segments)
+    segs = [segments[t] or [] for t in rids]
+    sample, bases, n = [], [], 0
+    for i in np.random.default_rng(0).permutation(len(rids)):
+        size = sum(len(x) for x in segs[i])
+        if n + size <= DUMP_SAMPLE_BASES:
+            sample.append(rids[i])
+            bases += segs[i]
+            n += size
+    out = {"target_ids": np.array(rids, np.float64), "segments_per_target": np.array([len(s) for s in segs], np.float64),
+           "segment_lengths": np.array([len(x) for s in segs for x in s], np.float64),
+           "sample_target_ids": np.array(sample, np.float64),
+           "sample_bases": np.frombuffer(b"".join(bases), np.uint8).astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
+def ensure_model():
+    """The benchmark's model blob, written to a temporary file (the tree may be read-only); the caller removes it."""
+    from herro_b200 import weights as hbw
+    fd, p = tempfile.mkstemp(prefix="herro_bench_model_", suffix=".hbw")
+    os.close(fd)
     cfg = hbw.NetConfig()
     hbw.save_blob(p, cfg, hbw.random_weights(cfg, seed=7))
     return p, cfg
@@ -272,6 +305,8 @@ def main():
                              "sample": f"{args.steps} steps x {per} target reads of the workload (CPU oracle on {threads} threads + torch fp32 "
                                        f"forward on {r['torch_threads']} intra-op threads, the fastest of a probe)"},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["segments"])
         os.remove(model)
         return
 
@@ -360,11 +395,12 @@ def main():
     assert r_e2e_w["checksum"] == r_e2e["checksum"], "hb_submit_alignments and hb_submit_target disagree"
     # one full-size launch (this rank's share of the last step), alone on the GPU: its per-kernel CUDA-event times feed the
     # roofline (in the pipelined region the lanes overlap, so per-kernel times there include the other lanes' kernels), and it
-    # is the launch the HBM-resident replay re-runs
+    # is the launch the HBM-resident replay re-runs; its corrected reads are what --dump-outputs writes
     ctx.reset_stats()
     ctx.set_launch_targets(lt)
     ctx.set_kernel_timing(True)
-    harness.run(cut[n_steps - 1], cut[n_steps], 1, harness.windowing(cut[n_steps - 1], cut[n_steps], wthr))  # same entry as `e2e`
+    r_full = harness.run(cut[n_steps - 1], cut[n_steps], 1, harness.windowing(cut[n_steps - 1], cut[n_steps], wthr),  # same entry as `e2e`
+                         collect=bool(args.dump_outputs) and rank == 0)
     st_full = ctx.stats()
     # ---- region 2: device stages only, inputs resident in HBM (one launch's working set is GBs of matrices + activations,
     #      larger than the 126 MB L2, so no L2 flush is needed)
@@ -376,6 +412,8 @@ def main():
     if rank == 0:
         sampler.join(timeout=3)
     st2 = ctx.stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {c.rid: c.segments for c in r_full["results"]})
     t_dev = ms_dev / 1e3
     vals = torch.tensor([t_dev, t_e2e, float(last_launch_bases * args.steps), float(r_e2e["bases"]), t_e2e_w, t_upload, t_gen,
                          float(st["host_allocs"]), float(st["windows"]), float(hi - lo)], dtype=torch.float64, device="cuda")

@@ -361,6 +361,8 @@ class Context:
 # C++ host harness (herro_b200/host/harness.cpp): the Rust binary's thread topology over the C ABI
 # ------------------------------------------------------------------------------------------
 _host = None
+# hbh_result_fn: (user, rid, seqs, seg_len, n_segs), called on the harness's consumer thread
+_RESULT_FN = C.CFUNCTYPE(None, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint8), C.POINTER(C.c_uint32), C.c_uint32)
 
 
 def _host_lib():
@@ -371,7 +373,7 @@ def _host_lib():
         vp, u32 = C.c_void_p, C.c_uint32
         H.hbh_pack_2bit.argtypes = [vp, vp, u32, vp, vp, C.c_int]
         H.hbh_windowing.argtypes = [vp, vp, vp, u32, u32, u32, C.c_int, vp, vp, C.c_uint64]
-        H.hbh_run.argtypes = [vp, vp, vp, vp, u32, u32, u32, C.c_int, vp, vp, vp, vp, vp, vp]
+        H.hbh_run.argtypes = [vp, vp, vp, vp, u32, u32, u32, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp]
         _host = H
     return _host
 
@@ -401,7 +403,8 @@ class HostHarness:
             raise HerroError(rc, "windowing failed")
         return ow, off
 
-    def run(self, t_begin: int, t_end: int, threads: int, windows=None) -> dict:
+    def run(self, t_begin: int, t_end: int, threads: int, windows=None, collect: bool = False) -> dict:
+        """collect: also return the corrected records the consumer polled, as `results` (list of Corrected)."""
         H = _host_lib()
         out3 = np.zeros(4, dtype=np.uint64)
         chk = C.c_uint64()
@@ -409,12 +412,25 @@ class HostHarness:
         sub = C.c_double()
         ow_p = windows[0].ctypes.data if windows is not None else None
         off_p = windows[1].ctypes.data if windows is not None else None
+        results = []
+
+        def keep(_user, rid, seqs, seg_len, n):
+            lens = [int(seg_len[k]) for k in range(n)]
+            data = C.string_at(seqs, sum(lens)) if n else b""
+            offs = np.cumsum([0] + lens)
+            results.append(Corrected(int(rid), [data[offs[k]:offs[k + 1]] for k in range(n)]))
+
+        cb = _RESULT_FN(keep) if collect else None  # alive until hbh_run returns
         rc = H.hbh_run(self.ctx._h, self.ovl.ctypes.data, self.aln_off.ctypes.data, self.read_len.ctypes.data,
-                       self.ctx.window_size, t_begin, t_end, threads, ow_p, off_p, out3.ctypes.data, C.byref(chk), C.byref(sec), C.byref(sub))
+                       self.ctx.window_size, t_begin, t_end, threads, ow_p, off_p, out3.ctypes.data, C.byref(chk), C.byref(sec), C.byref(sub),
+                       C.cast(cb, C.c_void_p) if cb is not None else None, None)
         if rc != 0:
             raise HerroError(rc, self.ctx._L.hb_last_error(self.ctx._h).decode())
-        return dict(bases=int(out3[0]), records=int(out3[1]), targets=int(out3[2]), failed=int(out3[3]), checksum=int(chk.value),
-                    seconds=sec.value, submit_seconds_sum=sub.value)
+        r = dict(bases=int(out3[0]), records=int(out3[1]), targets=int(out3[2]), failed=int(out3[3]), checksum=int(chk.value),
+                 seconds=sec.value, submit_seconds_sum=sub.value)
+        if collect:
+            r["results"] = results
+        return r
 
 
 # ------------------------------------------------------------------------------------------

@@ -97,9 +97,13 @@ int hbh_windowing(const hb_overlap* ovl_all, const uint64_t* aln_off, const uint
 // library window the alignments (hb_submit_alignments).  out4 = {corrected bases, records (segments),
 // targets that produced output, targets that failed (skipped, the run goes on)}; checksum = order-independent
 // hash of (rid, segment bytes).  Every thread binds itself to the NUMA node of the context's GPU.
+// on_result (may be NULL) sees every corrected record as hb_poll_corrected returned it, on the consumer thread,
+// before it is released.
+typedef void (*hbh_result_fn)(void* user, uint32_t rid, const uint8_t* seqs, const uint32_t* seg_len, uint32_t n_segs);
 int hbh_run(hb_ctx* ctx, const hb_overlap* ovl_all, const uint64_t* aln_off, const uint32_t* read_len, uint32_t window,
             uint32_t t_begin, uint32_t t_end, int threads, const hb_overlap_window* ow_all, const uint64_t* ow_off,
-            uint64_t* out3, uint64_t* checksum, double* seconds, double* submit_seconds_sum) {
+            uint64_t* out3, uint64_t* checksum, double* seconds, double* submit_seconds_sum, hbh_result_fn on_result,
+            void* user) {
     if (!ctx || !ovl_all || !aln_off || !read_len || !out3 || !seconds) return HB_ERR_ARG;
     std::atomic<uint32_t> next{t_begin};
     std::atomic<int> rc{0};
@@ -151,6 +155,7 @@ int hbh_run(hb_ctx* ctx, const hb_overlap* ovl_all, const uint64_t* aln_off, con
                 records += n;
                 targets += n ? 1 : 0;
                 sum += h;
+                if (on_result) on_result(user, rid, seqs, lens, n);
                 hb_release_result(ctx, seqs);
             } else if (r == 0) {
                 if (producers_left.load() == 0) {

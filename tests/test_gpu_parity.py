@@ -60,9 +60,11 @@ def test_host_harness_matches_python_path():
     h = api.HostHarness(ctx, rs.ovl9, rs.cigars, rs.cig_off, rs.aln_off, np.diff(rs.off).astype(np.uint32))
     r1 = h.run(0, rs.n, 4)                                   # library does the windowing
     r2 = h.run(0, rs.n, 3, h.windowing(0, rs.n, 2))          # host-computed windows
-    for r in (r1, r2):
+    r3 = h.run(0, rs.n, 2, h.windowing(0, rs.n, 2), collect=True)  # the records the consumer polled, kept
+    for r in (r1, r2, r3):
         assert r["bases"] == want_bases and r["targets"] == want_targets
-    assert r1["checksum"] == r2["checksum"]
+    assert r1["checksum"] == r2["checksum"] == r3["checksum"]
+    assert {c.rid: c.segments or None for c in r3["results"]} == a["segments"]
 
 
 def test_cli_fastq_oec_to_fasta(tmp_path):
